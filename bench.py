@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this framework on N B200s
     python bench.py --impl reference [...]                         # the reference's CPU path (oracle port)
+    python bench.py [...] --dump-outputs DIR                       # + what the last timed step computed, as DIR/*.npy
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL).  A "step" is one
 ``CycleGANModel.optimize_parameters()`` on a synthetic U(-1,1) 128^3 batch; rank 0 prints ONE JSON line.
@@ -262,6 +263,41 @@ def time_norm_kernels(torch, I, batch, hbm_peak, reps=10):
     return out
 
 
+DUMP_SAMPLE = 1 << 20       # --dump-outputs: elements kept of a larger output (4 MB in float32; 40 MB for a training step)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each (name, value) as <out_dir>/<name>.npy, tensors in float32 and Python floats in float64.  A
+    tensor of more than DUMP_SAMPLE elements is stored as a fixed seeded sample of its flattened (logical-layout)
+    values, the same indices on every run, so that the dumps of two builds compare element for element.  Two runs with
+    the same arguments dump identical values: the step adds its fp32 gradient partial sums in a fixed order
+    (wgrad_fixup_kernel, colsum_finish_kernel)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays:
+        if torch.is_tensor(v):
+            v = v.detach().reshape(-1)
+            if v.numel() > DUMP_SAMPLE:
+                idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+                v = v[idx.to(v.device)]
+            a = v.float().cpu().numpy()
+        else:
+            a = np.float64(v)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def step_outputs(model):
+    """What a training loop receives from the last optimize_parameters(): the losses, the generated volumes (the
+    visuals other than the inputs) and the updated weights of each network (its parameters, concatenated)."""
+    import torch
+    out = [("loss_" + k, v) for k, v in model.get_current_losses().items()]
+    out += [(k, v) for k, v in model.get_current_visuals().items() if not k.startswith("real_")]
+    for n in model.model_names:
+        out.append(("net_" + n, torch.cat([p.detach().reshape(-1) for p in getattr(model, "net" + n).parameters()])))
+    return out
+
+
 def load_traffic(kernel):
     """dram__bytes_read.sum + dram__bytes_write.sum per launch of the roofline kernel, from the committed
     `ncu --set full` capture (profiles/roofline_traffic.json); None when no capture of this kernel exists."""
@@ -323,8 +359,9 @@ def run_gpu(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms) / steps
 
-    def measure(batch, steps, warmup):
-        """(ms per resident step, ms per end-to-end step, kernels per step, host bytes per step) at one batch size."""
+    def measure(batch, steps, warmup, dump_dir=None):
+        """(ms per resident step, ms per end-to-end step, kernels per step, host bytes per step) at one batch size;
+        with dump_dir, rank 0 writes the outputs of the last resident step there before the end-to-end steps run."""
         g = torch.Generator().manual_seed(1234 + rank)
         shape = (batch, 1, PATCH, PATCH, PATCH)
         host_A = (torch.rand(shape, generator=g) * 2 - 1).pin_memory()
@@ -349,13 +386,15 @@ def run_gpu(args):
         graphs = getattr(model, "_graphs", None)
         if graphs and graphs.get("launches"):
             launches = graphs["launches"]               # replayed from the captured graphs: count taken at capture
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, step_outputs(model))
         ms_e2e = timed(step_e2e, steps)
         return ms_step, ms_e2e, int(launches), int(host_A.numel() * 4 * 2)
 
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_step, ms_e2e, launches, h2d = measure(per_gpu_batch, args.steps, args.warmup)
+    ms_step, ms_e2e, launches, h2d = measure(per_gpu_batch, args.steps, args.warmup, args.dump_outputs)
     clocks = sampler.stop() if sampler else None
     err = I.tc_error()
     if err:
@@ -501,6 +540,8 @@ def run_infer(args):
     l0 = I.launch_count()
     ms = timed(step_resident, args.steps)
     launches = (I.launch_count() - l0) // args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [("label", out["v"])])
     ms_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if sampler else None
     err = I.tc_error()
@@ -558,7 +599,13 @@ def main():
     ap.add_argument("--stride", type=int, default=32, help="--workload infer: window stride (reference default 32)")
     ap.add_argument("--windows-per-pass", type=int, default=4,
                     help="--workload infer: windows a rank sends through the generator as one batch (1 = the reference's loop)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last resident timed step computed (taken before the end-to-end steps) as "
+                         "DIR/<name>.npy (float32; outputs over %d elements as a fixed seeded sample), to compare two "
+                         "builds output for output" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU arm's outputs; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "infer":

@@ -158,10 +158,11 @@ int launch_naive_wgrad(NaiveWgradP P, cudaStream_t st) {
 }
 
 // dbias[c] += sum over rows of dy[row][c]   (rows = N*D*H*W)
+// Each block stores its partial sums in part[blockIdx.y][blockIdx.x][32]; colsum_finish_kernel adds them in block order,
+// so dbias is the same in every run (one fp32 atomicAdd per block summed them in timing order).
 template <typename T>
 __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ dy, long long rows, int C,
-                                                      float* __restrict__ out) {
-  // blockDim = 256 threads: thread handles channel (tid % C') ... generic scalar version
+                                                      float* __restrict__ part) {
   const int c = blockIdx.y * 32 + (threadIdx.x & 31);
   const int lane_row = threadIdx.x >> 5;           // 8 row lanes
   float acc = 0.f;
@@ -171,11 +172,27 @@ __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ dy, l
   __shared__ float sm[8][33];
   sm[lane_row][threadIdx.x & 31] = acc;
   __syncthreads();
-  if (lane_row == 0 && c < C) {
+  if (lane_row == 0) {
     float s = 0.f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) s += sm[i][threadIdx.x & 31];
-    atomicAdd(out + c, s);
+    part[((long long)blockIdx.y * gridDim.x + blockIdx.x) * 32 + threadIdx.x] = s;
+  }
+}
+__global__ void __launch_bounds__(256) colsum_finish_kernel(const float* __restrict__ part, int blocks, int C,
+                                                            float* __restrict__ out) {
+  // one warp per channel; lane l adds blocks l, l + 32, ... in order, then the 32 lane sums are added in lane order
+  const int c = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  __shared__ float sm[8][32];
+  float s = 0.f;
+  if (c < C)
+    for (int b = lane; b < blocks; b += 32) s += part[((long long)(c >> 5) * blocks + b) * 32 + (c & 31)];
+  sm[threadIdx.x >> 5][lane] = s;
+  __syncwarp();
+  if (c < C && lane == 0) {
+    float t = 0.f;
+    for (int i = 0; i < 32; ++i) t += sm[threadIdx.x >> 5][i];
+    out[c] += t;
   }
 }
 
@@ -185,9 +202,14 @@ int launch_colsum(const void* dy, long long rows, int C, float* out, cudaStream_
   long long bx = (rows + 8 * 64 - 1) / (8 * 64);
   if (bx > 1024) bx = 1024;
   if (bx < 1) bx = 1;
-  dim3 grid((unsigned)bx, (unsigned)((C + 31) / 32));
-  colsum_kernel<T><<<grid, 256, 0, st>>>(reinterpret_cast<const T*>(dy), rows, C, out);
+  const unsigned groups = (unsigned)((C + 31) / 32);
+  float* part = nullptr;                             // stream-ordered: capture-safe, freed after the finishing pass
+  MRA_CHECK_CUDA(cudaMallocAsync((void**)&part, (size_t)groups * bx * 32 * sizeof(float), st));
+  colsum_kernel<T><<<dim3((unsigned)bx, groups), 256, 0, st>>>(reinterpret_cast<const T*>(dy), rows, C, part);
   MRA_LAUNCH_CHECK();
+  colsum_finish_kernel<<<(unsigned)((C + 7) / 8), 256, 0, st>>>(part, (int)bx, C, out);
+  MRA_LAUNCH_CHECK();
+  MRA_CHECK_CUDA(cudaFreeAsync(part, st));
   return 0;
 }
 

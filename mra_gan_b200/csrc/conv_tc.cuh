@@ -805,6 +805,9 @@ __host__ __device__ constexpr uint32_t make_idesc_m(int m, int n) {
 // Scheduling is stream-K: the (work item x K-block) space, weighted by taps per item, is cut into
 // gridDim.x equal contiguous ranges (one CTA per SM, one wave); a CTA whose range crosses a work-item
 // boundary flushes its accumulators (fp32 red.global.add) and continues with the next item.
+// A work item that several CTAs share is not added piece by piece in timing order (fp32 addition is not associative, so dw
+// would change from run to run): each piece stores its partial tile in P.part, and wgrad_fixup_kernel adds the pieces of
+// the item to dw in K order once the launch is complete.  An item that one CTA does alone is added straight away.
 constexpr int kMaxWGroups = 4;
 struct WGroup {
   int tap0, ntaps;                  // range in the launch-ordered tap arrays
@@ -828,6 +831,8 @@ struct WgradP {
   long long total_cost;             // sum over work items of taps(item) * K-blocks
   float* dw;
   long long tap_stride, m_stride, n_stride;   // element strides of dw[tap][m][n] in memory
+  float* part;                      // partial tiles of shared items: [CTA][0: the piece that starts the CTA's range,
+  int part_cols;                    //   1: the piece that ends it][128 rows][part_cols]
   int* err;
   int stages;
   uint32_t tmem_cols;
@@ -1117,12 +1122,23 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmM, const __grid_constant__
       const int m = (kPair ? 2 * sg.mt + rank : sg.mt) * 128 + ml;
       const int n0 = sg.nt * ncols;
       const bool valid = ml < 64 * P.m_chunks && m < P.Km && !(P.debug & 1);
+      float* slot = nullptr;                               // a piece of a shared item: its partial tile, row ml
+      if (sg.kb0 > 0 || sg.kb1 < kblocks)
+        slot = P.part + (((long long)blockIdx.x * 2 + (sg.kb1 < kblocks ? 1 : 0)) * 128 + ml) * P.part_cols;
       for (int g = 0; g < sg.ntap; ++g) {
         float* obase = P.dw + (long long)P.twi[sg.tap0 + g] * P.tap_stride + (long long)m * P.m_stride;
         for (int c0 = 0; c0 < ncols; c0 += 32) {
           uint32_t r[32];
           tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(g * ncols + c0), r);
           tmem_wait_ld();
+          if (slot && P.n_stride != 1) {
+            float4* o = reinterpret_cast<float4*>(slot + g * ncols + c0);
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+              o[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
+                                 __uint_as_float(r[4 * j + 3]));
+            continue;
+          }
           if (P.n_stride == 1) {
             // A thread owns accumulator ROW ml and 32 consecutive columns = 128 B of one dw row; its neighbours' rows are
             // m_stride floats away, so a red.v4 straight from the registers touched 32 half-used sectors per warp
@@ -1143,7 +1159,9 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmM, const __grid_constant__
               const int row = i * 4 + (lane >> 3);                     // row of this warp's 32-row quadrant
               const int mr = q * 32 + row;
               const float4 v = stg[row * 8 + (ch ^ (row & 7))];
-              if (mr < 64 * P.m_chunks && m - ml + mr < P.Km && !(P.debug & 1)) {
+              if (slot) {                                              // a piece of a shared item: its partial tile
+                *reinterpret_cast<float4*>(slot + (long long)(mr - ml) * P.part_cols + g * ncols + c0 + ch * 4) = v;
+              } else if (mr < 64 * P.m_chunks && m - ml + mr < P.Km && !(P.debug & 1)) {
                 float* o = obase + (long long)(mr - ml) * P.m_stride + n0 + c0 + ch * 4;
                 asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(o), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
                              : "memory");
@@ -1439,6 +1457,67 @@ inline int run_gather_v1_launch(const GatherPlan& plan, const GatherLaunch* Ls, 
   return 0;
 }
 
+// Adds the pieces of every shared work item (blockIdx.x = work, blockIdx.y = slice of its elements) to dw in K order: the pieces are recomputed with the
+// stream-K arithmetic of wseg_begin / wseg_next, so that each is read from the slot its CTA stored it in.
+__global__ void __launch_bounds__(256) wgrad_fixup_kernel(const __grid_constant__ WgradP P, int nunits, int kctas) {
+  __shared__ int cta[160], which[160];
+  __shared__ int npieces;
+  const int per_item = P.m_tiles * P.n_tiles;
+  const int w = blockIdx.x;
+  const int item = w / per_item, rem = w - item * per_item;
+  const int g = wg_item_group(P, item);
+  const WGroup& G = P.grp[g];
+  const int ntap = wg_item_ntap(P, g, item);
+  const long long kblocks = (long long)P.tilesW * P.tilesH * P.tilesD * P.N;
+  if (threadIdx.x == 0) {
+    const long long works_full = (long long)(G.ntaps / G.gpi) * per_item, wl = w - (long long)G.item0 * per_item;
+    const long long W0 = G.cost0 + min(wl, works_full) * G.gpi * kblocks + max(wl - works_full, 0ll) * ntap * kblocks;
+    const long long W1 = W0 + ntap * kblocks;
+    const long long share = (P.total_cost + nunits - 1) / nunits;
+    int n = 0;
+    bool shared_item = false;
+    for (long long u = W0 / share; u * share < W1 && u < nunits && n < 160; ++u) {
+      const long long lo = max(W0, u * share), hi = min(W1, min((u + 1) * share, P.total_cost));
+      const long long kb0 = (lo - W0) / ntap, kb1 = hi == W1 ? kblocks : (hi - W0) / ntap;
+      if (kb1 <= kb0) continue;
+      if (kb0 > 0 || kb1 < kblocks) shared_item = true;
+      cta[n] = (int)u; which[n] = kb1 < kblocks ? 1 : 0; ++n;
+    }
+    npieces = shared_item ? n : 0;
+  }
+  __syncthreads();
+  const int np = npieces;
+  if (np == 0) return;
+  const int mt = rem / P.n_tiles, nt = rem - mt * P.n_tiles;
+  const int tap0 = G.tap0 + (item - G.item0) * G.gpi;
+  const int ncols = P.ncc * 64, nq = ncols / 4;            // four columns per thread: 16-byte loads
+  const int total = kctas * 128 * ntap * nq;
+  for (int e = blockIdx.y * blockDim.x + threadIdx.x; e < total; e += gridDim.y * blockDim.x) {
+    const int c = (e % nq) * 4;
+    int t = e / nq;
+    const int gg = t % ntap; t /= ntap;
+    const int ml = t % 128, rank = t / 128;
+    const int m = (kctas * mt + rank) * 128 + ml;
+    if (ml >= 64 * P.m_chunks || m >= P.Km) continue;
+    const long long off = (long long)ml * P.part_cols + gg * ncols + c;
+    const long long slot = 128ll * P.part_cols;
+    float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 4
+    for (int i = 0; i < np; ++i) {                           // K order: the loads may run ahead, the adds keep the order
+      const float4 v = __ldcg(reinterpret_cast<const float4*>(P.part + ((long long)(cta[i] * kctas + rank) * 2 + which[i]) * slot + off));
+      sum.x += v.x; sum.y += v.y; sum.z += v.z; sum.w += v.w;
+    }
+    float* o = P.dw + (long long)P.twi[tap0 + gg] * P.tap_stride + (long long)m * P.m_stride + (long long)(nt * ncols + c) * P.n_stride;
+    if (P.n_stride == 1) {
+      float4 d = *reinterpret_cast<float4*>(o);
+      d.x += sum.x; d.y += sum.y; d.z += sum.z; d.w += sum.w;
+      *reinterpret_cast<float4*>(o) = d;
+    } else {
+      o[0] += sum.x; o[P.n_stride] += sum.y; o[2 * P.n_stride] += sum.z; o[3 * P.n_stride] += sum.w;
+    }
+  }
+}
+
 // Tile geometry of a wgrad launch (K-block boxes, m / n tiles) and the CTA-pair decision; returns pair.
 inline bool wgrad_fill_geometry(const WgradPlan& plan, WgradP& P) {
   const bool sw = plan.m_is_shifted != 0;
@@ -1549,17 +1628,31 @@ inline int run_wgrad_tc(const WgradPlan& plan, const void* x, const void* dy, fl
   P.stages = stages;
   P.tmem_cols = pow2_cols(max_cols);
   const size_t smem = (size_t)stages * stage_bytes + 1024 + 256 + kWgradFlushBytes;
-  if (pair) {
-    MRA_CHECK_CUDA(launch_pdl(wgrad_tc_kernel<true>, dim3((unsigned)(num_sms() & ~1)), dim3(kThreads), smem, st, 2, tmM, maps, P));
-    MRA_LAUNCH_CHECK();
-    return 0;
-  }
-  // one wave: a CTA per SM (fewer when there is less than ~4 K-blocks of work per CTA)
-  long long ctas = num_sms();
-  if (P.total_cost < ctas * 4) ctas = (P.total_cost + 3) / 4;
+  // one wave: a CTA per SM (fewer when there is less than ~4 K-blocks of work per CTA); pairs: one unit per two SMs
+  long long ctas = pair ? (num_sms() & ~1) : num_sms();
+  if (!pair && P.total_cost < ctas * 4) ctas = (P.total_cost + 3) / 4;
   if (ctas < 1) ctas = 1;
-  MRA_CHECK_CUDA(launch_pdl(wgrad_tc_kernel<false>, dim3((unsigned)ctas), dim3(kThreads), smem, st, 1, tmM, maps, P));
+  const int kctas = pair ? 2 : 1, nunits = (int)(ctas / kctas);
+  MRA_REQUIRE(nunits <= 160, "wgrad: more stream-K units than the fixup kernel tracks");
+  bool shared_items = false;                         // does any work item span more than one unit?
+  for (int u = 0; u < nunits && !shared_items; ++u) {
+    WSegIter it; WSeg sg;
+    wseg_begin(P, kblocks, it, u, nunits);
+    while (wseg_next(P, kblocks, it, sg))
+      if (sg.kb0 > 0 || sg.kb1 < kblocks) { shared_items = true; break; }
+  }
+  P.part_cols = max_cols;
+  if (shared_items)                                  // stream-ordered: capture-safe, freed after the fixup
+    MRA_CHECK_CUDA(cudaMallocAsync((void**)&P.part, (size_t)ctas * 2 * 128 * max_cols * sizeof(float), st));
+  if (pair) MRA_CHECK_CUDA(launch_pdl(wgrad_tc_kernel<true>, dim3((unsigned)ctas), dim3(kThreads), smem, st, 2, tmM, maps, P));
+  else MRA_CHECK_CUDA(launch_pdl(wgrad_tc_kernel<false>, dim3((unsigned)ctas), dim3(kThreads), smem, st, 1, tmM, maps, P));
   MRA_LAUNCH_CHECK();
+  if (!shared_items) return 0;
+  // an item's elements are spread over many blocks: a few items may each hold up to one piece per unit
+  const unsigned slices = (unsigned)max(1ll, min(256ll, ((long long)kctas * 128 * max_cols / 4 + 255) / 256));
+  wgrad_fixup_kernel<<<dim3((unsigned)(P.n_items * P.m_tiles * P.n_tiles), slices), 256, 0, st>>>(P, nunits, kctas);
+  MRA_LAUNCH_CHECK();
+  MRA_CHECK_CUDA(cudaFreeAsync(P.part, st));
   return 0;
 }
 inline int run_wgrad_tc(const mra_conv_desc& d, const void* x, const void* dy, float* dw, cudaStream_t st) {

@@ -437,3 +437,11 @@ def synthetic_patches(batch, size, seed=1234, dtype=torch.float32):
 def rel_l2(a, b):
     a, b = a.double().flatten(), b.double().flatten()
     return float((a - b).norm() / (b.norm() + 1e-300))
+
+
+def golden_sample(t):
+    """What tests/golden/ stores of a network output, flattened: all of it up to 4096 elements, else every 5th element
+    (5 is odd, so on the power-of-two extents of the fixtures the sample visits every index of every axis).  This keeps
+    each fixture file under 1 MB."""
+    t = t.detach().reshape(-1)
+    return t if t.numel() <= 4096 else t[::5].clone()

@@ -3,7 +3,8 @@
     python -m oracle.make_golden
 
 Weights are synthetic and regenerated from seeds at test time (oracle.functional.make_weights);
-each fixture stores a checksum of them, the inputs' seeds and the REFERENCE's outputs.
+each fixture stores a checksum of them, the inputs' seeds and the REFERENCE's outputs (the larger ones as
+``OF.golden_sample``).
 """
 import os
 import random
@@ -107,8 +108,8 @@ def gen_batchnorm(nw):
         floor = dict(y=OF.rel_l2(y32.detach(), y.detach()), dx=OF.rel_l2(x32.grad, xi.grad),
                      grads=max(OF.rel_l2(g32[k].grad, v) for k, v in grads.items() if float(v.norm()) > 1e-12))
         out[name] = dict(weight_seed=seed, input_seed=7, checksum=OF.weights_checksum(sd), keys=list(sd.keys()),
-                         y=y.detach().float(), dx=xi.grad[:, :, ::2, ::2, ::2].float(), grads=grads, buffers=bufs,
-                         y_eval=y_eval.float(), fp32_floor=floor)
+                         y=OF.golden_sample(y.float()), dx=xi.grad[:, :, ::2, ::2, ::2].float(), grads=grads, buffers=bufs,
+                         y_eval=OF.golden_sample(y_eval.float()), fp32_floor=floor)
     return out
 
 
@@ -132,8 +133,8 @@ def gen_step(cycle_mod, no_lsgan, netG="resnet_9blocks", ngf=8, size=32, steps=2
             post = m.netG_A(A)   # train-mode forward, also EMA-updates running stats
         st = dict(input_seed=100 + s, losses=dict(m.get_current_losses()),
                   cor_coe_GA=float(m.loss_cor_coe_GA), cor_coe_GB=float(m.loss_cor_coe_GB),
-                  fake_B=m.fake_B.detach().clone(), rec_A=m.rec_A.detach().clone(),
-                  idt_A=m.idt_A.detach().clone(), post_G_A=post.clone())
+                  fake_B=OF.golden_sample(m.fake_B), rec_A=OF.golden_sample(m.rec_A),
+                  idt_A=OF.golden_sample(m.idt_A), post_G_A=OF.golden_sample(post))
         if s == 0:
             # fp64 "truth" for the post-step generator output (SURVEY.md section 4: compare errors against
             # fp64 instead of demanding agreement with one particular fp32 summation order)
@@ -145,7 +146,7 @@ def gen_step(cycle_mod, no_lsgan, netG="resnet_9blocks", ngf=8, size=32, steps=2
             with torch.no_grad():
                 post64 = o64.G("G_A", A.double())
             random.setstate(random_state)
-            st["post_G_A_fp64"] = post64.float()
+            st["post_G_A_fp64"] = OF.golden_sample(post64.float())
             st["ref_post_err_vs_fp64"] = float((post.double() - post64).abs().max())
             # gradients left in .grad after the step (G grads from backward_G, D from backward_D_*)
             g = {}
@@ -210,7 +211,7 @@ def gen_options(nw):
         y.square().mean().backward()
         out["pixel_ndf8_sig%d" % sig] = dict(weight_seed=41, weight_scale=0.3, input_seed=8, keys=list(spec.keys()),
                                              shapes=[tuple(v) for v in spec.values()], checksum=OF.weights_checksum(sd),
-                                             y=y.detach().clone(), dx=xi.grad.detach().clone(),
+                                             y=OF.golden_sample(y), dx=OF.golden_sample(xi.grad),
                                              dw0=net.state_dict(keep_vars=True)["net.0.weight"].grad.detach().clone())
     spec = OF.unet_g_spec(1, 1, 8, 2)
     sd = OF.make_weights(spec, 42, scale=0.2)

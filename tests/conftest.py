@@ -24,6 +24,18 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip_gpu)
 
 
+@pytest.fixture(autouse=True)
+def cpu_tests_build_on_the_cpu(request, monkeypatch):
+    """A test not marked gpu runs on the CPU also where a GPU is visible: networks and models are created on the CPU
+    (the package puts them on cuda whenever a GPU is present), as on a machine without one."""
+    if request.node.get_closest_marker("gpu") is None:
+        import torch
+        from mra_gan_b200 import networks3D
+        from mra_gan_b200.models import base_model
+        monkeypatch.setattr(networks3D, "device", torch.device("cpu"))
+        monkeypatch.setattr(base_model, "device", torch.device("cpu"))
+
+
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN

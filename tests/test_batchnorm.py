@@ -134,7 +134,7 @@ def _nets_vs_golden(golden_dir, dev, dtype, tol):
             x, _ = OF.synthetic_patches(2, 32, seed=r["input_seed"])
             xi = x.to(dev).requires_grad_(True)
             y = net(xi)
-            assert OF.rel_l2(y.detach().cpu(), r["y"]) < tol, name
+            assert OF.rel_l2(OF.golden_sample(y.detach().cpu()), r["y"]) < tol, name
             y.double().square().mean().backward()
             # gradients: the fixture is the reference in fp64; fp32_floor = the reference's own fp32 run against it (the
             # UNet's 1^3 bottleneck normalises 2 values per channel: 5e-3 on dx in fp32, whoever computes it)
@@ -154,7 +154,7 @@ def _nets_vs_golden(golden_dir, dev, dtype, tol):
             net.eval()
             with torch.no_grad():
                 ye = net(x.to(dev))
-            assert OF.rel_l2(ye.cpu(), r["y_eval"]) < tol, name
+            assert OF.rel_l2(OF.golden_sample(ye.cpu()), r["y_eval"]) < tol, name
     finally:
         N3.set_default_compute_dtype(torch.bfloat16)
 

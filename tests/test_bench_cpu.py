@@ -135,6 +135,55 @@ def test_default_batches_and_launch_modes(monkeypatch):
     assert bench.workload_config(1, 2, "eager")["model_tflop_per_sample_step"] == pytest.approx(48.54)
 
 
+def test_dump_outputs_of_a_training_step(tmp_path, monkeypatch):
+    """--dump-outputs: the eight losses (float64), the six generated volumes and the updated weights of the four networks
+    (float32) of the model's last step; an output over DUMP_SAMPLE elements as a sample that is the same on every run."""
+    import random
+
+    import numpy as np
+
+    from mra_gan_b200 import networks3D as N3
+    from mra_gan_b200 import ops
+    from mra_gan_b200.models import create_model
+    from oracle import functional as OF
+    from oracle.ops_ref import RefImpl
+    from oracle.ref_import import make_opt
+    # a training step dumps 10 tensors: at the full sample size they stay within 64 MB
+    assert 10 * bench.DUMP_SAMPLE * 4 <= 64 << 20
+    prev = ops.set_impl(RefImpl(torch.float32))
+    N3.set_default_compute_dtype(torch.float32)
+    try:
+        opt = make_opt(ngf=4, ndf=4, pool_size=2, checkpoints_dir=str(tmp_path))
+        random.seed(0)
+        m = create_model(opt)
+        m.setup(opt)
+        m.set_input(list(OF.synthetic_patches(1, 32, seed=1)))
+        m.optimize_parameters()
+        monkeypatch.setattr(bench, "DUMP_SAMPLE", 40000)    # the 32^3 volumes whole, the networks' weights sampled
+        for d in ("a", "b"):
+            bench.dump_outputs(str(tmp_path / d), bench.step_outputs(m))
+        losses = m.get_current_losses()
+        vols = ["fake_B", "rec_A", "idt_A", "fake_A", "rec_B", "idt_B"]
+        nets = ["G_A", "G_B", "D_A", "D_B"]
+        names = ["loss_" + k for k in losses] + vols + ["net_" + n for n in nets]
+        assert sorted(os.listdir(tmp_path / "a")) == sorted(n + ".npy" for n in names)
+        load = lambda d, n: np.load(str(tmp_path / d / (n + ".npy")))
+        for k, v in losses.items():
+            a = load("a", "loss_" + k)
+            assert a.dtype == np.float64 and a.shape == () and float(a) == v
+        for n in vols:
+            a = load("a", n)
+            assert a.dtype == np.float32 and np.array_equal(a, getattr(m, n).detach().reshape(-1).cpu().numpy())
+        for n in nets:
+            w = torch.cat([p.detach().reshape(-1) for p in getattr(m, "net" + n).parameters()]).cpu().numpy()
+            a = load("a", "net_" + n)
+            assert w.size > 40000 and a.dtype == np.float32 and a.shape == (40000,)
+            assert np.isin(a, w).all() and np.array_equal(a, load("b", "net_" + n))
+    finally:
+        ops.set_impl(prev)
+        N3.set_default_compute_dtype(torch.bfloat16)
+
+
 def test_gpu_arm_refuses_to_run_without_a_device():
     """No CPU fallback: without a CUDA device the GPU arm must fail loudly (non-zero exit, no JSON line)."""
     if torch.cuda.is_available():

@@ -112,10 +112,11 @@ def _infer_worker(rank, world, port, tmp, golden, q):
 
 
 @pytest.mark.timeout(600)
-def test_two_rank_sliding_window_reduces_to_the_reference_volume(golden_dir, tmp_path):
+def test_two_rank_sliding_window_reduces_to_the_reference_volume(golden_dir, tmp_path, monkeypatch):
     import torch.multiprocessing as mp
     r = torch.load(os.path.join(golden_dir, "sliding_window_small.pt"), weights_only=False)
     world, port = 2, _free_port()
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")     # the ranks run on the CPU also where a GPU is visible
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     procs = [ctx.Process(target=_infer_worker, args=(k, world, port, str(tmp_path), golden_dir, q)) for k in range(world)]

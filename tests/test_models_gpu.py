@@ -205,14 +205,15 @@ def test_cyclegan_step_matches_golden(golden_dir, case, mode, tmp_path):
     for k, v in st["losses"].items():
         assert got[k] == pytest.approx(v, rel=ltol, abs=1e-5), k
     assert float(m.loss_cor_coe_GA) == pytest.approx(st["cor_coe_GA"], rel=10 * ltol)
-    assert OF.rel_l2(m.fake_B.cpu(), st["fake_B"]) < atol and OF.rel_l2(m.rec_A.cpu(), st["rec_A"]) < 2 * atol
-    assert OF.rel_l2(m.idt_A.cpu(), st["idt_A"]) < atol
+    assert OF.rel_l2(OF.golden_sample(m.fake_B.cpu()), st["fake_B"]) < atol
+    assert OF.rel_l2(OF.golden_sample(m.rec_A.cpu()), st["rec_A"]) < 2 * atol
+    assert OF.rel_l2(OF.golden_sample(m.idt_A.cpu()), st["idt_A"]) < atol
     named = {"G_A": dict(m.netG_A.named_parameters()), "D_A": dict(m.netD_A.named_parameters())}
     for key, (nrm, samp) in st["grads"].items():
         net, pk = key.split(".", 1)
         assert float(named[net][pk].grad.double().norm()) == pytest.approx(nrm, rel=gtol), key
     with torch.no_grad():
-        post = m.netG_A(A.cuda()).cpu()
+        post = OF.golden_sample(m.netG_A(A.cuda()).cpu())
     err = float((post - st["post_G_A"]).abs().max())
     print("post-step max-abs G_A(real_A) error (%s, %s): %.3e" % (case, mode, err))
     if mode == "fp32":

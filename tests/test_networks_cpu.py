@@ -160,8 +160,9 @@ def test_cyclegan_step_matches_golden(golden_dir, case, tmp_path):
         for k, v in st["losses"].items():
             assert got[k] == pytest.approx(v, rel=ltol, abs=1e-6), k
         assert float(m.loss_cor_coe_GA) == pytest.approx(st["cor_coe_GA"], rel=10 * ltol)
-        assert OF.rel_l2(m.fake_B, st["fake_B"]) < atol and OF.rel_l2(m.rec_A, st["rec_A"]) < atol
-        assert OF.rel_l2(m.idt_A, st["idt_A"]) < atol
+        assert OF.rel_l2(OF.golden_sample(m.fake_B), st["fake_B"]) < atol
+        assert OF.rel_l2(OF.golden_sample(m.rec_A), st["rec_A"]) < atol
+        assert OF.rel_l2(OF.golden_sample(m.idt_A), st["idt_A"]) < atol
         if "grads" in st:
             named = {"G_A": dict(m.netG_A.named_parameters()), "D_A": dict(m.netD_A.named_parameters())}
             for key, (nrm, samp) in st["grads"].items():
@@ -170,7 +171,7 @@ def test_cyclegan_step_matches_golden(golden_dir, case, tmp_path):
         with torch.no_grad():
             post = m.netG_A(A)
         if si == 0:       # after ONE step (north_star); measured floor here ~2.5e-3, see DESIGN.md
-            assert float((post - st["post_G_A"]).abs().max()) < 1e-2
+            assert float((OF.golden_sample(post) - st["post_G_A"]).abs().max()) < 1e-2
     assert set(m.get_current_visuals()) == {"real_A", "fake_B", "rec_A", "idt_A", "real_B", "fake_A", "rec_B", "idt_B"}
 
 

@@ -117,6 +117,38 @@ def test_wgrad_cta_pair_path(monkeypatch):
     _check_conv(*case, torch.bfloat16, expect_tc=True)
 
 
+REPRO = [
+    (ConvGeom(256, 256, 3, 1, 0), (34, 34, 34), 2),        # G.rb at full size: CTA pairs, every item over several units
+    (ConvGeom(64, 128, 3, 2, 1), (64, 64, 64), 2),         # G.d1 at full size: four items, each over dozens of CTAs
+]
+
+
+@pytest.mark.parametrize("case", REPRO, ids=gid)
+def test_wgrad_and_dbias_are_bit_reproducible(case):
+    """A work item shared by several CTAs is added to dw in K order (wgrad_fixup_kernel) and the bias column sums in
+    block order: the same inputs give the same dw and db bit for bit, also when they are added into a gradient."""
+    I = ops.impl()
+    g, dims, n = case
+    x, _, _, dy = _conv_case(g, dims, n, torch.bfloat16)
+    xd, dyd = x.cuda(), dy.cuda()
+    dw, db = I.conv_wgrad(xd, dyd, g, want_bias=True)
+    base_w, base_b = torch.randn_like(dw), torch.randn_like(db)
+    acc = None
+    for _ in range(3):
+        w2, b2 = I.conv_wgrad(xd, dyd, g, want_bias=True)
+        assert torch.equal(w2, dw) and torch.equal(b2, db)
+        aw, ab = base_w.clone(), base_b.clone()
+        I.conv_wgrad(xd, dyd, g, want_bias=True, acc_dw=aw, acc_db=ab)
+        if acc is not None:
+            assert torch.equal(aw, acc[0]) and torch.equal(ab, acc[1])
+        acc = (aw, ab)
+    assert I.tc_error() == 0
+    if g.cin == 64:                                        # the fp64 reference of G.rb at 34^3 takes minutes on the host
+        dw_ref, db_ref = R.RefImpl(torch.float64).conv_wgrad(x.double(), dy.double(), g, want_bias=True)
+        assert rel_l2(dw.cpu(), dw_ref) < TOL[torch.bfloat16] and rel_l2(db.cpu(), db_ref) < TOL[torch.bfloat16]
+        assert rel_l2(acc[0].cpu() - base_w.cpu(), dw_ref) < TOL[torch.bfloat16]
+
+
 @pytest.mark.parametrize("case", TC_CONVS[:3], ids=gid)
 def test_conv_same_shape_fp32_path(case):
     _check_conv(*case, torch.float32, expect_tc=False)

@@ -73,11 +73,12 @@ def _worker(rank, world, port, tmp, q, fused):
 
 @pytest.mark.timeout(600)
 @pytest.mark.parametrize("fused", [False, True], ids=["autograd_accumulate", "fused_wgrad"])
-def test_two_rank_gradient_averaging_matches_batch_two(tmp_path, fused):
+def test_two_rank_gradient_averaging_matches_batch_two(tmp_path, fused, monkeypatch):
     """fused = True: the wgrad kernels add every use of a weight straight into its bucket view and the conv modules
     tell the buckets when a weight is final (MRA_DP_FUSED_WGRAD); every bucket must still go out exactly once, from
     inside the backward pass."""
     world, port = 2, _free_port()
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")     # the ranks run on the CPU also where a GPU is visible
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     procs = [ctx.Process(target=_worker, args=(r, world, port, str(tmp_path), q, fused)) for r in range(world)]

@@ -104,6 +104,18 @@ inline int num_sms() {
   return n;
 }
 
+// largest dynamic shared memory a block may opt into (cudaFuncAttributeMaxDynamicSharedMemorySize) on this device
+inline size_t max_optin_smem() {
+  static int n = 0;
+  if (!n) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&n, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess || n <= 0)
+      n = 48 * 1024;
+  }
+  return (size_t)n;
+}
+
 // ---- scalar / vector element access with fp32 math ----
 template <typename T> __device__ __forceinline__ float to_f(T v);
 template <> __device__ __forceinline__ float to_f<float>(float v) { return v; }

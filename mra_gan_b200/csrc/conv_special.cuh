@@ -320,21 +320,28 @@ inline int launch_expand_hw(const bf16* src, bf16* out, long long rows, int Hs, 
 // bands sized to the resident block count: rows = 256 planes (batch 2 x 128) on 148 x 6 slots -> 3 bands of 43 lines =
 // 768 items in one wave, instead of 1024 items of 32 lines in 2.3 waves.  A band re-reads the K - 1 Z lines it shares
 // with its neighbour (L2 hits).
+// Two line buffers of Wz positions x 33 words: 67.6 KB for the widest line the stem / head lowerings accept (256).
+inline size_t shift_sum_smem(int Wz) { return (size_t)2 * Wz * 33 * sizeof(uint32_t); }
 template <typename TO, int SGN, int K, bool CHECKW>
 inline int launch_shift_sum_t(const bf16* Z, TO* out, long long rows, int Hz, int Wz, int Ho, int Wo, int off, const float* bias,
                               int act, float slope, cudaStream_t st) {
   auto kern = shift_sum_kernel<TO, SGN, K, CHECKW>;
   int threads = ((Wo + 31) / 32) * 32;
   if (threads < 64) threads = 64;
-  const size_t smem = (size_t)2 * Wz * 33 * sizeof(uint32_t);          // two line buffers
-  MRA_REQUIRE(smem <= 48 * 1024, "shift_sum: Z line does not fit shared memory (Wz = %d)", Wz);
+  const size_t smem = shift_sum_smem(Wz);
+  MRA_REQUIRE(smem <= max_optin_smem(), "shift_sum: Z line does not fit shared memory (Wz = %d)", Wz);
   // resident blocks per SM for this (kernel, block size, shared memory): asked once per configuration (host-side query,
   // no stream work; the first call of a configuration happens in the eager warm-up steps, before any graph capture)
   static std::mutex mu;
   static std::map<std::pair<int, size_t>, int> occ_cache;
+  static bool attr_set = false;
   int occ = 0;
   {
     std::lock_guard<std::mutex> lk(mu);
+    if (!attr_set) {                                 // lines wider than 186 positions need more than the default 48 KB
+      MRA_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_optin_smem()));
+      attr_set = true;
+    }
     auto key = std::make_pair(threads, smem);
     auto it = occ_cache.find(key);
     if (it == occ_cache.end()) {
@@ -586,6 +593,7 @@ inline int stem_wgrad(const mra_conv_desc& d, const void* x, const void* dy, flo
 }
 
 inline int stem_dgrad(const mra_conv_desc& d, const void* dy, const void* wT, void* dx, void* wsp, size_t wsb, cudaStream_t st) {
+  MRA_REQUIRE(shift_sum_smem(d.wout) <= max_optin_smem(), "stem dgrad: Z line does not fit shared memory (W = %d)", d.wout);
   Workspace ws{(char*)wsp, wsb, 0};
   const long long rows = (long long)d.n * d.din;
   MRA_WS_TAKE(Z, bf16, (size_t)rows * d.hout * d.wout * 64 * 2);                    // bf16, see head_fprop
@@ -602,6 +610,7 @@ inline int stem_dgrad(const mra_conv_desc& d, const void* dy, const void* wT, vo
 
 inline int head_fprop(const mra_conv_desc& d, const void* x, const void* w, const float* bias, void* y, void* wsp, size_t wsb,
                       cudaStream_t st) {
+  MRA_REQUIRE(shift_sum_smem(d.win) <= max_optin_smem(), "head fprop: Z line does not fit shared memory (W = %d)", d.win);
   Workspace ws{(char*)wsp, wsb, 0};
   const long long rows = (long long)d.n * d.dout;
   // Z (the per-(kh,kw) partial sums over kd and ci) is stored in bf16: its 49 terms per output are summed in fp32

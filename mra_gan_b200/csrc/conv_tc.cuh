@@ -1285,6 +1285,11 @@ inline bool gather_eligible(const mra_conv_desc& d, int which) {
   if (ck % 64 != 0 || pick_n_tile(cn) == 0) return false;
   if (d.k * d.k * d.k > kMaxTaps) return false;
   if (d.stride != 1 && d.stride != 2) return false;
+  // the strided "dgrad form" (Conv3d dgrad, ConvTranspose3d fprop) runs one launch per parity phase of the output; with
+  // k < stride some phases have no tap at all (their dx is zero, their y the bias alone), and the gather kernels only
+  // write the positions of the phases they run
+  const bool direct = (which == 0) != (d.transposed != 0);
+  if (!direct && d.k < d.stride) return false;
   return true;
 }
 inline bool wgrad_eligible(const mra_conv_desc& d) {

@@ -97,10 +97,22 @@ int mra_conv3d_fprop(const mra_conv_desc* d, const void* x, const void* w, const
   cudaStream_t st = (cudaStream_t)stream;
   if (stats) MRA_CHECK_CUDA(cudaMemsetAsync(stats, 0, sizeof(double) * 2 * d->n * d->cout, st));
   if (special::im2col_eligible(*d)) return special::im2col_fprop(*d, x, w, bias, y, stats, workspace, workspace_bytes, st);
-  if (special::convT1_eligible(*d) && !stats)
-    return special::im2col_dgrad(special::convT1_mirror(*d), x, w, y, workspace, workspace_bytes, st, bias, d->act, d->slope);
   if (special::stem_eligible(*d)) return special::stem_fprop(*d, x, w, bias, y, stats, workspace, workspace_bytes, st);
-  if (special::head_eligible(*d) && !stats) return special::head_fprop(*d, x, w, bias, y, workspace, workspace_bytes, st);
+  if (special::convT1_eligible(*d) || special::head_eligible(*d)) {
+    // single-channel outputs: no epilogue statistics in these lowerings, so they come from a pass over the stored y
+    MRA_REQUIRE(!stats || d->act == MRA_ACT_NONE, "stats are defined on the pre-activation output only");
+    if (special::convT1_eligible(*d)) {
+      if (int rc = special::im2col_dgrad(special::convT1_mirror(*d), x, w, y, workspace, workspace_bytes, st, bias, d->act, d->slope))
+        return rc;
+    } else if (int rc = special::head_fprop(*d, x, w, bias, y, workspace, workspace_bytes, st)) {
+      return rc;
+    }
+    if (!stats) return 0;
+    mra_norm_desc nd;
+    memset(&nd, 0, sizeof(nd));
+    nd.n = d->n; nd.c = d->cout; nd.d = d->dout; nd.h = d->hout; nd.w = d->wout; nd.res_pad = -1; nd.dtype = d->dtype;
+    return mra_inorm_stats(&nd, y, stats, stream);
+  }
   if (tc::gather_eligible(*d, 0)) {
     bool split = false;
     if (int rc = tc::run_gather_tc(*d, 0, x, w, bias, y, stats, st, nullptr, 0.f, workspace, workspace_bytes, &split)) return rc;

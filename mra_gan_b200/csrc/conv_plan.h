@@ -203,7 +203,7 @@ inline bool build_wgrad_plan(const GeomEx& d, WgradPlan& P) {
   for (int kd = 0; kd < d.k[0]; ++kd) for (int kh = 0; kh < d.k[1]; ++kh) for (int kw = 0; kw < d.k[2]; ++kw)
     P.taps.push_back(Tap{kd - d.pad[0], kh - d.pad[1], kw - d.pad[2], (kd * d.k[1] + kh) * d.k[2] + kw});
   choose_box(P.qdims, 64, 256 / s, P.box);
-  // ---- launch structure (tensor-core kernel only; needs 64-channel multiples) ----
+  // ---- launch structure (tensor-core kernel only; channel counts in 64-channel chunks) ----
   P.launches.clear();
   const int cs = d.transposed ? d.cout : d.cin;          // channels of the shifted operand
   P.ncc = cs % 256 == 0 ? 4 : (cs % 128 == 0 ? 2 : 1);

@@ -403,11 +403,11 @@ struct Workspace {
 
 inline bool stem_eligible(const mra_conv_desc& d) {
   return d.dtype == MRA_BF16 && !(d.flags & MRA_CONV_FORCE_NAIVE) && !d.transposed && d.stride == 1 && d.pad == 0 &&
-         d.cin == 1 && d.k >= 2 && d.k <= 8 && d.win <= 256 && tc::pick_n_tile(d.cout) > 0;
+         d.cin == 1 && d.k >= 2 && d.k <= 8 && d.win <= 256 && tc::tc_channels_ok(d.cout);
 }
 inline bool head_eligible(const mra_conv_desc& d) {
   return d.dtype == MRA_BF16 && !(d.flags & MRA_CONV_FORCE_NAIVE) && !d.transposed && d.stride == 1 && d.pad >= 0 &&
-         d.pad < d.k && d.cout == 1 && d.k >= 2 && d.k <= 8 && d.win <= 256 && d.cin % 64 == 0;
+         d.pad < d.k && d.cout == 1 && d.k >= 2 && d.k <= 8 && d.win <= 256 && tc::tc_channels_ok(d.cin);
 }
 
 inline bool im2col_eligible(const mra_conv_desc& d) {
@@ -415,7 +415,7 @@ inline bool im2col_eligible(const mra_conv_desc& d) {
   if ((long long)d.n * d.dout * d.hout * d.wout * 8 >= (1ll << 32) || (long long)d.n * d.din * d.hin * d.win >= (1ll << 31))
     return false;
   return d.dtype == MRA_BF16 && !(d.flags & MRA_CONV_FORCE_NAIVE) && !d.transposed && d.cin == 1 &&
-         d.k * d.k * d.k <= 64 && tc::pick_n_tile(d.cout) > 0 && !(d.stride == 1 && d.pad == 0 && d.k >= 2);
+         d.k * d.k * d.k <= 64 && tc::tc_channels_ok(d.cout) && !(d.stride == 1 && d.pad == 0 && d.k >= 2);
 }
 // ConvTranspose3d(C -> 1, k, s, p) (the UNet's outermost up-convolution, networks3D.py:312-316) is, operand for operand,
 // the mirror Conv3d(1 -> C, k, s, p) with the roles of x and y swapped:

@@ -695,18 +695,22 @@ gather_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                               (long long)(lh * P.ostep + P.ph_oh[t.ph]) * P.osh +
                               (long long)(lw * P.ostep + P.ph_ow[t.ph]) * P.osw + t.n0;
       if (kMode != 0 && (t.n != st_n || t.n0 != st_n0)) {
-        epilogue_flush_stats(P.stats, st_n, P.Cn, st_n0, W.q, W.c_begin, 2, nchunks, lane, st, defer, d1, d2, epi_red);
+        epilogue_flush_stats(P.stats, st_n, P.Cn, st_n0, W.q, W.c_begin, 2, min(nchunks, (P.Cn - st_n0) >> 5), lane, st, defer,
+                             d1, d2, epi_red);
         st_n = t.n; st_n0 = t.n0;
       }
+      // chunks of the tile that hold output channels: all of them unless Cn is not a multiple of the tile width (then the
+      // last N tile stops at Cn; paired phases need Cn == 64, i.e. whole tiles)
+      const int tchunks = P.pair ? acc_cols / 32 : min(acc_cols / 32, (P.Cn - t.n0) >> 5);
       AuxRegs ax;
-      epilogue_aux_first<kMode>(E, W.c_begin, acc_cols / 32, valid, obase, P.pair != 0, ax);
+      epilogue_aux_first<kMode>(E, W.c_begin, tchunks, valid, obase, P.pair != 0, ax);
       ok = mbar_wait(&acc_full[buf], aph, P.err, 3);
       if (!ok) break;
       tc_fence_after();
       const long long te0 = (P.debug & 2) ? clock64() : 0;
       const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * acc_cols);
       uint64_t* rel_bar = &acc_empty[buf];
-      epilogue_tile<kMode>(E, t_addr, W.c_begin, 2, acc_cols / 32, valid, obase, t.n0, lane, st, 0, defer, d1, d2, ax, [&]() {
+      epilogue_tile<kMode>(E, t_addr, W.c_begin, 2, tchunks, valid, obase, t.n0, lane, st, 0, defer, d1, d2, ax, [&]() {
         tc_fence_before();                      // accumulator fully read: hand the buffer back to the MMA warp
         __syncwarp();
         if (lane == 0) mbar_arrive(rel_bar);
@@ -714,7 +718,9 @@ gather_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       if ((P.debug & 2) && threadIdx.x == 0) atomicAdd(P.dbg + 4, (unsigned long long)(clock64() - te0));
       if (++buf == P.nbuf) { buf = 0; aph ^= 1u; }
     }
-    if (kMode != 0) epilogue_flush_stats(P.stats, st_n, P.Cn, st_n0, W.q, W.c_begin, 2, nchunks, lane, st, defer, d1, d2, epi_red);
+    if (kMode != 0)
+      epilogue_flush_stats(P.stats, st_n, P.Cn, st_n0, W.q, W.c_begin, 2, min(nchunks, (P.Cn - st_n0) >> 5), lane, st, defer, d1,
+                           d2, epi_red);
   }
   tc_fence_before();
   __syncthreads();
@@ -1128,6 +1134,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmM, const __grid_constant__
       for (int g = 0; g < sg.ntap; ++g) {
         float* obase = P.dw + (long long)P.twi[sg.tap0 + g] * P.tap_stride + (long long)m * P.m_stride;
         for (int c0 = 0; c0 < ncols; c0 += 32) {
+          if (n0 + c0 >= P.Kn) break;                      // columns past the shifted operand's channels (Kn % 64 == 32)
           uint32_t r[32];
           tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(g * ncols + c0), r);
           tmem_wait_ld();
@@ -1278,11 +1285,20 @@ inline int pick_n_tile(int cn) {
   if (cn % 64 == 0) return 64;
   return 0;
 }
+// Channel counts the tensor-core kernels accept on either side of a GEMM: multiples of 32.  A count that is not a multiple
+// of 64 (32, 96, 160, ...) still moves in 64-channel boxes: on the reduction side the box's upper half lies past the
+// tensor's channel extent and TMA fills it with zeros; on the output side the last 64-wide N tile is masked in the
+// epilogue / wgrad flush (columns >= Cn are computed from zero or unrelated operand rows and never stored).  Only the
+// per-tap gather kernel and the wgrad kernel take such shapes (run_gather_tc): the halo, column, phase and split-K
+// kernels keep their multiple-of-64 requirements.
+inline bool tc_channels_ok(int c) { return c > 0 && c % 32 == 0; }
+inline bool tc_channels_c64(int c) { return c % 64 == 0; }
+inline int gather_n_tile(int cn) { return pick_n_tile(cn) > 0 ? pick_n_tile(cn) : (tc_channels_ok(cn) ? 64 : 0); }
 
 inline bool gather_eligible(const mra_conv_desc& d, int which) {
   if (d.dtype != MRA_BF16 || (d.flags & MRA_CONV_FORCE_NAIVE)) return false;
   const int ck = which == 0 ? d.cin : d.cout, cn = which == 0 ? d.cout : d.cin;
-  if (ck % 64 != 0 || pick_n_tile(cn) == 0) return false;
+  if (!tc_channels_ok(ck) || !tc_channels_ok(cn)) return false;
   if (d.k * d.k * d.k > kMaxTaps) return false;
   if (d.stride != 1 && d.stride != 2) return false;
   // the strided "dgrad form" (Conv3d dgrad, ConvTranspose3d fprop) runs one launch per parity phase of the output; with
@@ -1294,7 +1310,7 @@ inline bool gather_eligible(const mra_conv_desc& d, int which) {
 }
 inline bool wgrad_eligible(const mra_conv_desc& d) {
   if (d.dtype != MRA_BF16 || (d.flags & MRA_CONV_FORCE_NAIVE)) return false;
-  if (d.cout % 64 != 0 || d.cin % 64 != 0) return false;
+  if (!tc_channels_ok(d.cout) || !tc_channels_ok(d.cin)) return false;
   if (d.k * d.k * d.k > kMaxTaps) return false;
   if (d.stride != 1 && d.stride != 2) return false;
   return true;
@@ -1392,7 +1408,7 @@ inline int run_gather_v1_launch(const GatherPlan& plan, const GatherLaunch* Ls, 
   P.Dl = L.dims[0]; P.Hl = L.dims[1]; P.Wl = L.dims[2];
   P.tilesD = (P.Dl + P.bd - 1) / P.bd; P.tilesH = (P.Hl + P.bh - 1) / P.bh; P.tilesW = (P.Wl + P.bw - 1) / P.bw;
   P.astep = L.astep;
-  P.Cn = plan.cn; P.n_tile = n_tile; P.n_tiles = plan.cn / n_tile; P.kchunks = plan.ck / 64;
+  P.Cn = plan.cn; P.n_tile = n_tile; P.n_tiles = (plan.cn + n_tile - 1) / n_tile; P.kchunks = (plan.ck + 63) / 64;
   const long long total_tiles = (long long)plan.n * P.tilesD * P.tilesH * P.tilesW * P.n_tiles * items;
   MRA_REQUIRE(total_tiles < (1ll << 31), "too many tiles");
   P.total_tiles = (int)total_tiles;
@@ -1503,7 +1519,7 @@ __global__ void __launch_bounds__(256) wgrad_fixup_kernel(const __grid_constant_
     const int gg = t % ntap; t /= ntap;
     const int ml = t % 128, rank = t / 128;
     const int m = (kctas * mt + rank) * 128 + ml;
-    if (ml >= 64 * P.m_chunks || m >= P.Km) continue;
+    if (ml >= 64 * P.m_chunks || m >= P.Km || nt * ncols + c >= P.Kn) continue;
     const long long off = (long long)ml * P.part_cols + gg * ncols + c;
     const long long slot = 128ll * P.part_cols;
     float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1532,7 +1548,7 @@ inline bool wgrad_fill_geometry(const WgradPlan& plan, WgradP& P) {
   P.tilesW = (plan.qdims[2] + P.bw - 1) / P.bw;
   P.N = plan.n; P.sstep = plan.sstep;
   P.Km = Km; P.Kn = Kn;
-  P.m_chunks = Km >= 128 ? 2 : 1;
+  P.m_chunks = Km > 64 ? 2 : 1;                             // 64-channel boxes (Km = 96: the second one half zero-filled)
   P.ncc = plan.ncc;
   // CTA pairs (cta_group::2): 256 dense channels per unit, each CTA loads half of the shifted chunks.  Needs whole
   // 256-channel m tiles and one tap per MMA (ncc == 4), and enough K-blocks to feed 74 pairs.
@@ -1541,7 +1557,7 @@ inline bool wgrad_fill_geometry(const WgradPlan& plan, WgradP& P) {
   const bool pair = Km % 256 == 0 && plan.ncc == 4 && (num_sms() % 2) == 0 && getenv("MRA_WGRAD_NOPAIR") == nullptr &&
                     (long long)plan.qdims[0] * plan.qdims[1] * plan.qdims[2] * plan.n >= pair_min;
   P.m_tiles = pair ? Km / 256 : (Km + 127) / 128;
-  P.n_tiles = Kn / (64 * P.ncc);
+  P.n_tiles = (Kn + 64 * P.ncc - 1) / (64 * P.ncc);
   return pair;
 }
 // The stream-K side of a wgrad launch: tap groups -> work items -> cost prefixes (needs P.m_tiles / P.n_tiles).  Kept apart
@@ -1569,7 +1585,7 @@ inline bool wgrad_fill_schedule(const WgradPlan& plan, long long kblocks, WgradP
 }
 inline int run_wgrad_tc(const WgradPlan& plan, const void* x, const void* dy, float* dw, cudaStream_t st) {
   int* err = tc_err_flag();
-  MRA_REQUIRE(plan.cm % 64 == 0 && plan.cn % 64 == 0 && (int)plan.taps.size() <= kMaxTaps,
+  MRA_REQUIRE(tc_channels_ok(plan.cm) && tc_channels_ok(plan.cn) && (int)plan.taps.size() <= kMaxTaps,
               "shape not eligible for the tensor-core wgrad path");
   MRA_REQUIRE(!plan.launches.empty() && (int)plan.launches.size() <= kMaxWGroups, "wgrad plan: bad group count");
   static bool attr_set = false;

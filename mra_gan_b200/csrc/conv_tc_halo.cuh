@@ -592,10 +592,12 @@ inline bool phase_try_run(const GatherPlan& plan, const GatherRun& R, cudaStream
 
 // Run every launch of a gather plan on the tensor cores: the 8 parity phases of a stride-2 dgrad-form plan on the
 // phase-halo kernel, stride-1 launches on the halo-plane kernel, the rest (and anything those cannot host) on the
-// per-tap kernel.
+// per-tap kernel.  Channel counts that are multiples of 32 but not of 64 run on the per-tap kernel only (see
+// tc_channels_ok): its K chunks come zero-filled from TMA and its epilogue masks the N tile at Cn.
 inline int run_gather_tc(const GatherPlan& plan, const GatherRun& R, cudaStream_t st) {
-  const int n_tile = pick_n_tile(plan.cn);
-  MRA_REQUIRE(n_tile > 0 && plan.ck % 64 == 0, "channel counts not eligible for the tensor-core path");
+  const int n_tile = gather_n_tile(plan.cn);
+  MRA_REQUIRE(n_tile > 0 && tc_channels_ok(plan.ck), "channel counts not eligible for the tensor-core path");
+  const bool c64 = tc_channels_c64(plan.ck) && tc_channels_c64(plan.cn);
   const long long rows = (long long)R.slabs * plan.cn;
   CUtensorMap tmB;
   if (int rc = make_weight_map(&tmB, R.b, rows, plan.ck, n_tile)) return rc;
@@ -604,9 +606,10 @@ inline int run_gather_tc(const GatherPlan& plan, const GatherRun& R, cudaStream_
   const bool force_v1 = gm && !strcmp(gm, "v1");
   const bool no_pair = gm && !strcmp(gm, "single");
   const bool no_col = gm && !strcmp(gm, "nocol");
+  const bool plane_kernels = !force_v1 && c64;             // phase, column and halo kernels
   if (!force_v1 && gather_mergeable(plan)) {
     int prc = 0;
-    if (!(gm && !strcmp(gm, "nophase")) && phase_try_run(plan, R, st, &prc)) return prc;
+    if (c64 && !(gm && !strcmp(gm, "nophase")) && phase_try_run(plan, R, st, &prc)) return prc;
     bool slabs_ok = true;
     for (const GatherLaunch& L : plan.launches)
       for (const Tap& t : L.taps) if (t.widx >= R.slabs) slabs_ok = false;
@@ -617,7 +620,7 @@ inline int run_gather_tc(const GatherPlan& plan, const GatherRun& R, cudaStream_
     for (const Tap& t : L.taps) if (t.widx >= R.slabs) slabs_ok = false;
     ColP CP;
     memset(&CP, 0, sizeof(CP));
-    if (!force_v1 && !no_col && slabs_ok && col_setup(L, plan.n, plan.ck, plan.cn, CP)) {
+    if (plane_kernels && !no_col && slabs_ok && col_setup(L, plan.n, plan.ck, plan.cn, CP)) {
       if (int rc = run_gather_col(plan, L, CP, R, tmB, st)) return rc;
       continue;
     }
@@ -630,7 +633,7 @@ inline int run_gather_tc(const GatherPlan& plan, const GatherRun& R, cudaStream_
       if (t.dw < lo[1]) lo[1] = t.dw; if (t.dw > hi[1]) hi[1] = t.dw;
     }
     const bool reuse = !L.taps.empty() && (hi[0] - lo[0] + 1) * (hi[1] - lo[1] + 1) >= 4;
-    bool halo = !force_v1 && reuse && halo_setup(L, plan.n, plan.ck, plan.cn, !no_pair, P);
+    bool halo = plane_kernels && reuse && halo_setup(L, plan.n, plan.ck, plan.cn, !no_pair, P);
     if (halo) for (const Tap& t : L.taps) if (t.widx >= R.slabs) halo = false;
     if (halo) { if (int rc = run_gather_halo(plan, L, P, R, tmB, st)) return rc; }
     else      { if (int rc = run_gather_v1_launch(plan, &L, 1, R, tmB, n_tile, st)) return rc; }

@@ -513,7 +513,8 @@ int mra_debug_schedule(const mra_conv_desc* d, int which, int units, int single,
   if (which == 2) {
     WgradPlan plan;
     MRA_REQUIRE(build_wgrad_plan(*d, plan), "unsupported geometry");
-    MRA_REQUIRE(plan.cm % 64 == 0 && plan.cn % 64 == 0 && !plan.launches.empty(), "shape not eligible for the tensor-core wgrad path");
+    MRA_REQUIRE(tc::tc_channels_ok(plan.cm) && tc::tc_channels_ok(plan.cn) && !plan.launches.empty(),
+                "shape not eligible for the tensor-core wgrad path");
     tc::WgradP P;
     memset(&P, 0, sizeof(P));
     const bool pair = tc::wgrad_fill_geometry(plan, P);
